@@ -3,6 +3,11 @@
 
   python bench.py --gpus N --steps K --warmup W            # this repository's CUDA path
   python bench.py --impl reference --gpus N --steps K ...   # reference-semantics CPU path (oracle) on host cores
+  python bench.py ... --dump-outputs DIR                    # also write one step of the timed path as DIR/*.npy
+
+Every timed region of GPU train steps is exactly K steps.  Inputs and initial weights are seeded; --dump-outputs
+writes what one step of the timed path computes from the seeded weights, so that two builds run with the same
+arguments can be compared output for output.
 
 Workload (BASELINE.json configs[1]): Alibaba-trace-shaped synthetic batch, 256 DAGs x 200 nodes / 600 edges,
 64-dim, num_layers=3 (3 TransformerConv + 2 BN), fp32, per GPU (weak scaling for N > 1: every rank trains on
@@ -394,34 +399,57 @@ def _workload_string(cfg, B):
             f"num_layers={c['num_layers']}, fwd+bwd+Adam")
 
 
-def timed_blocks(run_block, K, barrier, world, dev, min_region_s=0.6, max_blocks=300, min_blocks=5):
-    """Times R blocks of EXACTLY K steps each (barrier + synchronize on both sides of every block, CUDA events around
-    it, max over ranks per block) and returns (median seconds per block, list of block seconds).  R is chosen so that
-    the whole timed region lasts >= min_region_s: a 13 ms region (20 steps of 0.67 ms) gives NVML no samples and lets
-    one scheduler hiccup move the headline by percents."""
+def timed_steps(run_block, K, barrier, world, dev):
+    """Seconds taken by EXACTLY K steps: barrier + synchronize on both sides, a CUDA event pair around the K steps, max
+    over ranks."""
     import torch.distributed as dist
 
-    def one():
-        barrier()
-        e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
-        e0.record()
-        run_block(K)
-        e1.record()
-        barrier()
-        return e0.elapsed_time(e1) * 1e-3
+    barrier()
+    e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
+    e0.record()
+    run_block(K)
+    e1.record()
+    barrier()
+    secs = e0.elapsed_time(e1) * 1e-3
+    if world > 1:
+        t = torch.tensor([secs], device=dev)
+        dist.all_reduce(t, op=dist.ReduceOp.MAX)
+        secs = float(t)
+    return secs
 
-    est = one()
-    if world > 1:
-        t = torch.tensor([est], device=dev)
-        dist.all_reduce(t, op=dist.ReduceOp.MAX)
-        est = float(t)
-    R = int(min(max_blocks, max(min_blocks, -(-min_region_s // max(est, 1e-6)))))
-    secs = [one() for _ in range(R)]
-    if world > 1:
-        t = torch.tensor(secs, device=dev)
-        dist.all_reduce(t, op=dist.ReduceOp.MAX)
-        secs = t.tolist()
-    return statistics.median(secs), secs
+
+def dump_step(out_dir, step, opt, fp, model, init, batch):
+    """Runs ``step``, one step of the timed path (graph replay of forward + backward, then Adam), on ``batch`` from
+    the seeded initial state ``init`` -- parameters, BatchNorm buffers, fresh Adam moments -- and, when ``out_dir`` is
+    set, writes what it hands its caller as float .npy files: the loss, the flat gradient buffer it computed, the flat
+    parameter buffer after the Adam update (the engine's own layout, one 256-byte-aligned slot per parameter) and the
+    BatchNorm buffers.  Collective for N > 1; only rank 0 passes ``out_dir``.
+    A step from fixed inputs is what can be compared: the kernels accumulate some sums with float atomics, so two runs
+    differ in the last bits of every step, and over many steps Adam (whose first updates are ~lr * sign(gradient))
+    and the BatchNorm ReLUs amplify that -- two identical trainings on one B200 differed in their gradients by 4e-6
+    after one step, 1e-3 after two and 5e-2 after fifteen.  Two runs of this dump (cfg2, one B200) agreed on the loss
+    exactly, on the gradients to 6e-8 of the largest and on the parameters to 4e-5 of the largest; that last figure
+    is the lin_skip.bias in front of each BatchNorm, whose gradient is zero in exact arithmetic (rounding noise of
+    1e-8) and which Adam's first update moves by up to lr regardless; every other parameter agreed within 2e-6."""
+    import numpy as np
+
+    with torch.no_grad():
+        fp.flat.copy_(init["flat"])
+        opt.m.zero_()
+        opt.v.zero_()
+        opt.t = 0
+        for n, b in model.named_buffers():
+            b.copy_(init[n])
+    loss = step(batch)
+    torch.cuda.synchronize()
+    if out_dir is None:
+        return
+    arrays = {"loss": loss, "grads": fp.grad, "params": fp.flat}
+    arrays.update({f"buffer.{n}": b for n, b in model.named_buffers()})
+    os.makedirs(out_dir, exist_ok=True)
+    for name, t in arrays.items():
+        a = t.detach().cpu().numpy()
+        np.save(os.path.join(out_dir, name + ".npy"), a.astype(np.float32 if a.dtype == np.float32 else np.float64))
 
 
 def first_step_parity(model, batch_host, dev, tau=0.5):
@@ -516,6 +544,7 @@ def run_b200(args, rank, world, local_rank):
     fp = FlatParams(model)
     opt, grad_sync = make_optimizer(fp)
     dp = DataParallel(fp) if world > 1 else None
+    init = {"flat": fp.flat.clone(), **{n: b.clone() for n, b in model.named_buffers()}}
 
     # ---- kernel-only arm: inputs resident in HBM -------------------------------------------------
     # The step is replayed from a CUDA graph per resident batch (train.GraphedTrainStep: index build + forward +
@@ -544,12 +573,13 @@ def run_b200(args, rank, world, local_rank):
     l0 = ops.LAUNCHES["n"]
     s0 = state["i"]
     t_wall = time.perf_counter()
-    secs, blocks = timed_blocks(resident_block, args.steps, barrier, world, dev)
+    secs = timed_steps(resident_block, args.steps, barrier, world, dev)
     t_wall = time.perf_counter() - t_wall
     launches_per_step = (ops.LAUNCHES["n"] - l0) / max(1, state["i"] - s0)
     clocks = sampler.stop() if rank == 0 else None
     peer_phases = opt.phase_times_us(reset=True) if hasattr(opt, "phase_times_us") and world > 1 else None
-    loss = state["loss"]
+    loss = float(state["loss"])          # read now: the dumped step below reuses the graph's loss buffer
+    last_batch = dev_batches[(state["i"] - 1) % N_ROT]
     value = world * B * args.steps / secs
 
     # ---- in-step kernel durations: the engine records a caller-created CUDA event pair around ONE kernel family of
@@ -592,7 +622,7 @@ def run_b200(args, rank, world, local_rank):
             st2["i"] += 1
 
     dropin_block(args.warmup)
-    secs2, _ = timed_blocks(dropin_block, args.steps, barrier, world, dev, min_region_s=0.3, max_blocks=40)
+    secs2 = timed_steps(dropin_block, args.steps, barrier, world, dev)
     e2e_val = world * B * args.steps / secs2
 
     # ---- end-to-end through the fused public API: pinned host batch -> device -> graph-replayed step -> loss read-back
@@ -615,7 +645,7 @@ def run_b200(args, rank, world, local_rank):
         return total + (v if v is not None else 0.0)
 
     fused_block(max(args.warmup, 9))
-    secs3, _ = timed_blocks(fused_block, args.steps, barrier, world, dev)
+    secs3 = timed_steps(fused_block, args.steps, barrier, world, dev)
     e2e_fused_val = world * B * args.steps / secs3
 
     # ---- BASELINE.json configs[3] (4096 graphs over 8 GPUs = 512 graphs / GPU, 128-dim, 3 layers) beside the headline
@@ -628,6 +658,8 @@ def run_b200(args, rank, world, local_rank):
         except Exception as e:  # noqa: BLE001 -- a supplementary block must not take the headline line down
             pert_pipe = {"error": repr(e)[:300]}
 
+    if args.dump_outputs:
+        dump_step(args.dump_outputs if rank == 0 else None, stepper, opt, fp, model, init, last_batch)
     if hasattr(opt, "check"):
         opt.check()
     if rank != 0:
@@ -678,10 +710,8 @@ def run_b200(args, rank, world, local_rank):
                    "step_issue": ("CUDA-graph replay per batch buffer (index build + forward + loss + backward), eager "
                                   f"all-reduce + Adam; {gstep.replays} replays, capture_error={gstep.capture_error}")
                    if use_graph else "eager fused_train_step (5 C calls per step)",
-                   "timing": f"{len(blocks)} blocks of exactly {args.steps} steps, each bracketed by barrier + "
-                             "synchronize and a CUDA event pair, max over ranks per block; value = median block "
-                             f"(min {min(blocks) * 1e3:.3f} / max {max(blocks) * 1e3:.3f} ms per block, timed region "
-                             f"{sum(blocks):.2f} s)",
+                   "timing": f"exactly {args.steps} steps bracketed by barrier + synchronize and a CUDA event pair, "
+                             f"max over ranks (timed region {secs:.3f} s)",
                    "l2": f"rotating {N_ROT} distinct resident batches; ~{(n_convs * 8 * Nn * H * 4) >> 20} MB of "
                          "activations written+read per step (> 126 MB L2 for cfg2+): no explicit flush in the step "
                          "loop; scatter_max is timed with an explicit 512 MB L2 flush"},
@@ -739,8 +769,8 @@ def run_extra_block(args, rank, world, dev, barrier, make_optimizer, cfg, per_gp
     barrier()
     if hasattr(opt, "phase_times_us"):
         opt.phase_times_us(reset=True)
-    K = max(5, min(args.steps, 20))
-    secs, blocks = timed_blocks(block, K, barrier, world, dev, min_region_s=0.4, max_blocks=60)
+    K = args.steps
+    secs = timed_steps(block, K, barrier, world, dev)
     phases = opt.phase_times_us(reset=True) if hasattr(opt, "phase_times_us") and world > 1 else None
     if hasattr(opt, "check"):
         opt.check()
@@ -748,7 +778,7 @@ def run_extra_block(args, rank, world, dev, barrier, make_optimizer, cfg, per_gp
         opt.close()
     Nn, Ee = batches[0].x.size(0), batches[0].edge_index.size(1)
     return {"workload": workload, "value": world * per_gpu * K / secs, "unit": "DAGs/s", "global_batch": world * per_gpu,
-            "ms_per_step": 1e3 * secs / K, "steps_per_block": K, "blocks": len(blocks), "nodes_per_gpu": Nn,
+            "ms_per_step": 1e3 * secs / K, "steps": K, "nodes_per_gpu": Nn,
             "edges_per_gpu": Ee, "grad_sync": sync, "peer": phases, "replays": gstep.replays,
             "capture_error": gstep.capture_error}
 
@@ -803,8 +833,8 @@ def run_pert_pipeline_block(args, dev, barrier):
 
     epoch_block(5)
     barrier()
-    K = max(5, min(args.steps, 20))
-    secs, blocks = timed_blocks(epoch_block, K, barrier, 1, dev, min_region_s=0.3, max_blocks=40)
+    K = args.steps
+    secs = timed_steps(epoch_block, K, barrier, 1, dev)
     store.check()
     res = [store.assemble(ids[i * B:(i + 1) * B]) for i in range(3)]
     gstep = GraphedTrainStep(model, opt, 0.5, None)
@@ -817,7 +847,7 @@ def run_pert_pipeline_block(args, dev, barrier):
 
     block(7)
     barrier()
-    secs2, blocks2 = timed_blocks(block, K, barrier, 1, dev, min_region_s=0.3, max_blocks=40)
+    secs2 = timed_steps(block, K, barrier, 1, dev)
     Nn, Ee = int(res[0].x.size(0)), int(res[0].edge_index.size(1))
     return {"workload": f"PERT-exact synthetic: {B} traces per step, one PERT graph each (60-72 calls: nodes = 2 calls + "
                         "distinct ms, edges = 4 calls), 64-dim, num_layers=3, fwd+bwd+Adam",
@@ -826,11 +856,11 @@ def run_pert_pipeline_block(args, dev, barrier):
                             "patterns_per_s": info2["patterns"] / info2["build_s"],
                             "what": "host span rows -> H2D -> count + build kernels -> level index -> node_depth"},
             "from_trace_ids": {"value": B * K / secs, "unit": "DAGs/s", "ms_per_step": 1e3 * secs / K,
-                               "h2d_bytes_per_step": 8 * B, "blocks": len(blocks),
+                               "h2d_bytes_per_step": 8 * B,
                                "what": "device-side sample assembly + collation from the resident store, then the eager "
                                        "fused train step"},
             "resident_graph_replay": {"value": B * K / secs2, "unit": "DAGs/s", "ms_per_step": 1e3 * secs2 / K,
-                                      "blocks": len(blocks2), "replays": gstep.replays,
+                                      "replays": gstep.replays,
                                       "capture_error": gstep.capture_error},
             "nodes_per_batch": Nn, "edges_per_batch": Ee, "store_resident_bytes": store.resident_bytes}
 
@@ -845,6 +875,9 @@ def main():
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-parity-check", action="store_true")
     ap.add_argument("--no-cfg4", action="store_true")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write what one step of the timed path computes from the seeded "
+                         "weights on the last timed batch (loss, gradients, updated parameters) to DIR")
     args = ap.parse_args()
     global _BENCH_CFG
     _BENCH_CFG = args.cfg
