@@ -47,7 +47,8 @@ extern "C" {
 
 /* ABI version (major*1000 + minor).  2000: pert_tconv_bwd takes rpc_ws; node_depth / eval-metric entry points.
  * 2001: pert_pert_graph_count / pert_pert_graph_build.  2002: pert_allreduce_adam timing[5], reduce-scatter form.
- * 2003: pert_span_graph_count / pert_span_graph_build. */
+ * 2003: pert_span_graph_count / pert_span_graph_build.  2004: training-mode dropout in the step engine
+ * (pert_model_forward gains dropout_p + rng_state, pert_model_backward gains dropout_p), pert_dropout_mask. */
 int pert_version(void);
 
 /* ---- index construction (integer, bit-exact) ---------------------------------------------------
@@ -159,6 +160,16 @@ int pert_bn_bwd(const float* dy, int ld_dy, const float* y, int ld_y, const floa
                 const float* rstd, const float* gamma, int relu, int training, float* dx, int ld_dx, float* dgamma,
                 float* dbeta, float* sums, long long N, int H, void* stream);
 
+/* ---- dropout after BatchNorm+ReLU (model.py:103, F.dropout(p, training)) ------------------------------------------
+ * The step engine applies dropout inside the BatchNorm-apply kernel with a counter-based generator, so no mask is
+ * stored: Philox4x32-10 with key = (seed & 0xffffffff, seed >> 32) and counter = (j & 0xffffffff, j >> 32, layer,
+ * offset), where j = n * (H/4) + c/4 is the float4 index of unit (n, c) of the [N, H] output of BatchNorm `layer`;
+ * output word c % 4 drops the unit iff it is < floor(p * 2^32) (computed in double; p = 1 drops everything).  Kept
+ * units are scaled by 1/(1-p) in fp32.  Test / debug aid: writes that keep mask, keep[n*H + c] = 1 (kept) or 0, for
+ * the given (seed, offset, layer).  p NaN or outside [0, 1] -> PERT_ERR_BADARG. */
+int pert_dropout_mask(long long seed, long long offset, int layer, long long N, int H, float p, uint8_t* keep,
+                      void* stream);
+
 /* ---- local head + probability-weighted add-pool (model.py:105-107) -----------------------------------
  * local[n] = <x_n, w_local> + b_local (skipped when local NULL);
  * pool[batch[n], :] += (x_n * probs[n]) / pnn[n]   (pool [B,H] is zeroed by the call). */
@@ -255,7 +266,7 @@ long long pert_model_workspace_offset(const PertModelDesc* desc, long long N, lo
 /* Optional measurement probe: the engine records the two caller-created cudaEvent_t around ONE kernel family of ONE
  * layer, on the launching stream (bench.py: in-step duration of the dominant kernel).  kernel: 1 = fused conv forward,
  * 2 = fused conv backward (target + source pass), 3 = node-linear forward GEMM, 4 = weight-gradient GEMM,
- * 5 = data-gradient GEMM.  NULL = no probe. */
+ * 5 = data-gradient GEMM, 6 = BatchNorm apply (+ fused dropout) of BatchNorm `layer`.  NULL = no probe. */
 typedef struct PertProbe {
   int32_t kernel, layer;
   void* ev_start;
@@ -265,17 +276,23 @@ int pert_model_forward(const PertModelDesc* desc, const float* params, float* bn
                        const float* x, const int64_t* cat_X, const int64_t* entry_id, const float* probs,
                        const float* pnn, const int64_t* batch, long long N, long long E, long long B,
                        const int* rowptr, const int* csr_src, const int* csr_if, const int* csr_rpc, void* workspace,
-                       long long workspace_bytes, int training, float* global_pred, float* local_pred, int* status,
-                       const PertProbe* probe, void* index_ready, void* stream);
+                       long long workspace_bytes, int training, float dropout_p, long long* rng_state,
+                       float* global_pred, float* local_pred, int* status, const PertProbe* probe, void* index_ready,
+                       void* stream);
 /* index_ready: optional cudaEvent_t recorded (on another stream) after the graph index was built: the forward waits
  * for it only right before the first attention kernel, so the index build overlaps the parameter pack, the input
  * prologue and the first GEMM.  NULL = the index is already complete in `stream` order.
- * Must follow pert_model_forward on the same workspace.  d_global [B], d_local [N] or NULL. */
+ * dropout_p in [0, 1] (else PERT_ERR_BADARG before any launch): with training and dropout_p > 0 every BatchNorm+ReLU
+ * output is passed through dropout (see pert_dropout_mask for the mask).  rng_state: caller-owned device int64[2] =
+ * (seed, offset), read by the BatchNorm kernels; the forward then adds 1 to the offset ON THE DEVICE after the last of
+ * them, so a replayed CUDA graph draws fresh masks on every replay.  May be NULL when training == 0 or dropout_p == 0.
+ * Must follow pert_model_forward on the same workspace, with the same training / dropout_p.  d_global [B], d_local [N]
+ * or NULL. */
 int pert_model_backward(const PertModelDesc* desc, const float* params, float* grads, const int64_t* cat_X,
                         const int64_t* entry_id, const float* probs, const float* pnn, const int64_t* batch,
                         long long N, long long E, long long B, const int* rowptr, const int* csr_src,
                         const int* csr_if, const int* csr_rpc, const int* colptr, const int* csc_pos,
-                        const int* csc_dst, void* workspace, long long workspace_bytes, int training,
+                        const int* csc_dst, void* workspace, long long workspace_bytes, int training, float dropout_p,
                         const float* d_global, const float* d_local, const PertProbe* probe, void* stream);
 
 /* ---- device-side batch assembly from a resident pattern store (csrc/store.cu) ---------------------------------------

@@ -64,8 +64,10 @@ SIGNATURES = {
     "pert_model_workspace_bytes": (LL, [P, LL, LL, LL]),
     "pert_model_packed_bytes": (LL, [P]),
     "pert_model_workspace_offset": (LL, [P, LL, LL, LL, I, I]),
-    "pert_model_forward": (I, [P, P, P, P, P, P, P, P, P, P, LL, LL, LL, P, P, P, P, P, LL, I, P, P, P, P, P, P]),
-    "pert_model_backward": (I, [P, P, P, P, P, P, P, P, LL, LL, LL, P, P, P, P, P, P, P, P, LL, I, P, P, P, P]),
+    "pert_model_forward": (I, [P, P, P, P, P, P, P, P, P, P, LL, LL, LL, P, P, P, P, P, LL, I, F, P, P, P, P, P, P,
+                               P]),
+    "pert_model_backward": (I, [P, P, P, P, P, P, P, P, LL, LL, LL, P, P, P, P, P, P, P, P, LL, I, F, P, P, P, P]),
+    "pert_dropout_mask": (I, [LL, LL, I, LL, I, F, P, P]),
 }
 
 _lib = None

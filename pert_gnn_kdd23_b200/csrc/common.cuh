@@ -52,6 +52,45 @@ __device__ __forceinline__ float group_sum(float v, unsigned gmask) {
   return v;
 }
 
+// ---------------------------------------------------------------- dropout masks (counter-based, no stored state)
+// Philox4x32-10 (Salmon et al., SC'11; the Random123 constants).  Pure function of (counter, key): any unit's mask can
+// be recomputed from (seed, offset, layer, position) alone -- by the backward pass, by pert_dropout_mask and by the
+// numpy restatement the tests compare against -- and does not depend on the launch geometry.
+__device__ __forceinline__ uint4 philox4x32_10(uint4 c, uint2 k) {
+#pragma unroll
+  for (int r = 0; r < 10; ++r) {
+    if (r) {
+      k.x += 0x9E3779B9u;
+      k.y += 0xBB67AE85u;
+    }
+    const uint32_t hi0 = __umulhi(0xD2511F53u, c.x), lo0 = 0xD2511F53u * c.x;
+    const uint32_t hi1 = __umulhi(0xCD9E8D57u, c.z), lo1 = 0xCD9E8D57u * c.z;
+    c = make_uint4(hi1 ^ c.y ^ k.x, lo1, hi0 ^ c.w ^ k.y, lo0);
+  }
+  return c;
+}
+// The four words that decide columns 4*(j % (H/4)) + 0..3 of row j / (H/4) of an [N, H] activation:
+// key = (seed lo, seed hi), counter = (j lo, j hi, layer, offset).  Unit k is dropped iff word k < t.
+__device__ __forceinline__ uint4 dropout_words(unsigned long long seed, unsigned long long offset, int layer,
+                                               unsigned long long j) {
+  return philox4x32_10(make_uint4((uint32_t)j, (uint32_t)(j >> 32), (uint32_t)layer, (uint32_t)offset),
+                       make_uint2((uint32_t)seed, (uint32_t)(seed >> 32)));
+}
+struct PertDropout {            // by-value kernel argument of the fused BatchNorm-apply dropout
+  const long long* rng;         // device (seed, offset), caller-owned
+  unsigned long long t;         // drop iff word < t;  t = floor(p 2^32)  (2^32 at p = 1: everything dropped)
+  float scale;                  // 1 / (1 - p);  0 at p = 1
+  int layer;
+};
+// host: threshold and scale of a dropout probability; false if p is NaN or outside [0, 1]
+static inline bool pert_dropout_params(float p, unsigned long long* t, float* scale) {
+  if (!(p >= 0.f && p <= 1.f)) return false;
+  const double pd = (double)p;
+  *t = (unsigned long long)floor(pd * 4294967296.0);
+  *scale = p == 1.f ? 0.f : (float)(1.0 / (1.0 - pd));
+  return true;
+}
+
 // engine-internal entry points (not part of the C-ABI)
 struct PertTiles {            // graph-aligned tile list of one batch for one row width (csrc/tconv_tile.cu)
   const int* tile_ptr;        // [*ntiles + 1] node boundaries (device)
@@ -78,4 +117,8 @@ int pert_tconv_bwd_tiles(const float* g, int ld_g, const float* q, const float* 
 int pert_bn_fwd_ex(const float* x, int ld_x, const float* gamma, const float* beta, float* running_mean,
                    float* running_var, long long* num_batches_tracked, float eps, float momentum, int training,
                    int relu, float* mean, float* rstd, float* y, int ld_y, long long N, int H, void* workspace,
-                   long long workspace_bytes, int stats_ready, void* stream);
+                   long long workspace_bytes, int stats_ready, float dropout_p, const long long* rng_state,
+                   int layer, void* stream);
+int pert_bn_bwd_ex(const float* dy, int ld_dy, const float* y, int ld_y, const float* x, int ld_x, const float* mean,
+                   const float* rstd, const float* gamma, int relu, int training, float dropout_scale, float* dx,
+                   int ld_dx, float* dgamma, float* dbeta, float* sums, long long N, int H, void* stream);

@@ -188,8 +188,11 @@ __global__ void __launch_bounds__(HEAD_T) k_head_fwd(const float* __restrict__ p
                                                      const float* __restrict__ W1, const float* __restrict__ b1,
                                                      const float* __restrict__ W2, const float* __restrict__ b2,
                                                      float* __restrict__ z, float* __restrict__ h1,
-                                                     float* __restrict__ out, int B, int H, int* status) {
+                                                     float* __restrict__ out, int B, int H, int* status,
+                                                     long long* rng_state) {
   extern __shared__ float hs[];                       // W1t [2H][H] | z [HEAD_G][2H]
+  // dropout: every BatchNorm apply of this forward has finished (stream order) -> advance the offset for the next one
+  if (rng_state && blockIdx.x == 0 && threadIdx.x == 0) rng_state[1] += 1;
   float* w1t = hs;
   float* zs_all = hs + (size_t)2 * H * H;
   const int w = threadIdx.x >> 5, lane = threadIdx.x & 31;
@@ -246,6 +249,9 @@ __global__ void __launch_bounds__(HEAD_T) k_head_fwd(const float* __restrict__ p
   for (int off = 16; off > 0; off >>= 1) o += __shfl_xor_sync(0xffffffffu, o, off);
   if (lane == 0) out[b] = o + __ldg(b2);
 }
+
+// the offset advance of k_head_fwd for a batch without graphs (B == 0: no head launch)
+__global__ void k_rng_advance(long long* rng_state) { rng_state[1] += 1; }
 
 // Backward of the head for HEAD_G graphs per CTA: dh1 = dg W2 (h1 > 0); dz = dh1 W1 -> dpool | entry-embedding rows
 // (atomic scatter); dW2 += dg h1; db2 += dg; dW1 += dh1^T z; db1 += dh1 (block-level sums, then one atomic per value).
@@ -592,9 +598,13 @@ int pert_model_forward(const PertModelDesc* d, const float* params, float* bn_ru
                        const float* x, const int64_t* cat_X, const int64_t* entry_id, const float* probs,
                        const float* pnn, const int64_t* batch, long long N, long long E, long long B,
                        const int* rowptr, const int* csr_src, const int* csr_if, const int* csr_rpc, void* workspace,
-                       long long workspace_bytes, int training, float* global_pred, float* local_pred, int* status,
-                       const PertProbe* probe, void* index_ready, void* stream) {
+                       long long workspace_bytes, int training, float dropout_p, long long* rng_state,
+                       float* global_pred, float* local_pred, int* status, const PertProbe* probe, void* index_ready,
+                       void* stream) {
   TRY(check_desc(d));
+  if (!(dropout_p >= 0.f && dropout_p <= 1.f)) return PERT_ERR_BADARG;
+  const bool drop = training && dropout_p > 0.f;
+  if (drop && !rng_state) return PERT_ERR_BADARG;
   std::lock_guard<std::mutex> issue_lock(engine_mutex());
   if (!params || !x || !cat_X || !entry_id || !probs || !pnn || !batch || !rowptr || !workspace || !global_pred)
     return PERT_ERR_BADARG;
@@ -676,10 +686,13 @@ int pert_model_forward(const PertModelDesc* d, const float* params, float* bn_ru
     if (l + 1 < L) {
       float* rm = bn_running ? bn_running + (size_t)l * 2 * H : nullptr;
       float* rv = rm ? rm + H : nullptr;
+      PROBE_START(6, l);
       TRY(pert_bn_fwd_ex(w.out[l], H, params + d->off_bn_g[l], params + d->off_bn_b[l], rm, rv,
                          (training && bn_nbt) ? bn_nbt + l : nullptr, d->bn_eps, d->bn_momentum, training, 1,
                          w.bn_stats[l], w.bn_stats[l] + H, w.x[l + 1], H, N, H, w.bn_part,
-                         pert_bn_workspace_bytes(N, H), stats_fused, st));
+                         pert_bn_workspace_bytes(N, H), stats_fused, drop ? dropout_p : 0.f,
+                         drop ? rng_state : nullptr, l, st));
+      PROBE_STOP(6, l);
     }
   }
   // 4. local head + weighted add-pool, global head
@@ -693,7 +706,10 @@ int pert_model_forward(const PertModelDesc* d, const float* params, float* bn_ru
     }
     k_head_fwd<<<pert_cdiv(B, HEAD_G), HEAD_T, hsm, st>>>(
         w.pool, params + d->off_entry, d->n_entry, entry_id, params + d->off_g1_w, params + d->off_g1_b,
-        params + d->off_g2_w, params + d->off_g2_b, w.z, w.h1, global_pred, (int)B, H, status);
+        params + d->off_g2_w, params + d->off_g2_b, w.z, w.h1, global_pred, (int)B, H, status,
+        drop ? rng_state : nullptr);
+  } else if (drop) {
+    k_rng_advance<<<1, 1, 0, st>>>(rng_state);
   }
   PERT_LAUNCH_CHECK();
   return PERT_OK;
@@ -704,9 +720,13 @@ int pert_model_backward(const PertModelDesc* d, const float* params, float* grad
                         const int64_t* entry_id, const float* probs, const float* pnn, const int64_t* batch,
                         long long N, long long E, long long B, const int* rowptr, const int* csr_src,
                         const int* csr_if, const int* csr_rpc, const int* colptr, const int* csc_pos,
-                        const int* csc_dst, void* workspace, long long workspace_bytes, int training,
+                        const int* csc_dst, void* workspace, long long workspace_bytes, int training, float dropout_p,
                         const float* d_global, const float* d_local, const PertProbe* probe, void* stream) {
   TRY(check_desc(d));
+  unsigned long long drop_t;
+  float drop_scale;
+  if (!pert_dropout_params(dropout_p, &drop_t, &drop_scale)) return PERT_ERR_BADARG;
+  if (!(training && dropout_p > 0.f)) drop_scale = 1.f;
   std::lock_guard<std::mutex> issue_lock(engine_mutex());
   if (!params || !grads || !cat_X || !entry_id || !probs || !pnn || !batch || !rowptr || !colptr || !workspace ||
       !d_global)
@@ -786,9 +806,10 @@ int pert_model_backward(const PertModelDesc* d, const float* params, float* grad
     PROBE_STOP(5, l);
     if (l > 0) {
       // BN(+ReLU) backward of layer l-1: dx (grad wrt x[l]) -> g of conv l-1, into the skip plane
-      TRY(pert_bn_bwd(w.dx, K, w.x[l], H, w.out[l - 1], H, w.bn_stats[l - 1], w.bn_stats[l - 1] + H,
-                      params + d->off_bn_g[l - 1], 1, training, dskip, H, grads + d->off_bn_g[l - 1],
-                      grads + d->off_bn_b[l - 1], w.sums, N, H, st));
+      // (with dropout, x[l] is the post-dropout output: x[l] > 0 <=> kept and active; dz = dx * scale there)
+      TRY(pert_bn_bwd_ex(w.dx, K, w.x[l], H, w.out[l - 1], H, w.bn_stats[l - 1], w.bn_stats[l - 1] + H,
+                         params + d->off_bn_g[l - 1], 1, training, drop_scale, dskip, H, grads + d->off_bn_g[l - 1],
+                         grads + d->off_bn_b[l - 1], w.sums, N, H, st));
     }
   }
   if (forked) TRY(aux_join(ax, st));

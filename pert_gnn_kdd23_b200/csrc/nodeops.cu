@@ -150,12 +150,16 @@ __global__ void k_bn_eval_stats(const float* __restrict__ rm, const float* __res
 // y = (relu)((x - mean) rstd gamma + beta).  acc != null (training): mean / rstd come from the fp64 sums of
 // k_bn_partial (every CTA derives them in its prologue; CTA 0 also stores them for the backward pass and updates the
 // running statistics); acc == null (eval): mean / rstd arrays are read.
+// DROP (training dropout, p > 0): y *= keep * scale in the same pass, keep from dropout_words(seed, offset, layer, j)
+// with j = the float4 index n * H/4 + c/4 -- exactly `id` below.  DROP = false is the plain kernel, no Philox in it.
+template <bool DROP>
 __global__ void __launch_bounds__(256) k_bn_apply(const float* __restrict__ x, int ld_x, float* __restrict__ mean,
                                                    float* __restrict__ rstd, const float* __restrict__ gamma,
                                                    const float* __restrict__ beta, float* __restrict__ y, int ld_y,
                                                    long long N, int H, int relu, const double* __restrict__ acc,
                                                    float eps, float momentum, float* running_mean,
-                                                   float* running_var, long long* num_batches_tracked) {
+                                                   float* running_var, long long* num_batches_tracked,
+                                                   PertDropout dr) {
   extern __shared__ float s_par[];   // mean | rstd | gamma | beta
   for (int c = threadIdx.x; c < H; c += blockDim.x) {
     float mu, rs;
@@ -187,6 +191,11 @@ __global__ void __launch_bounds__(256) k_bn_apply(const float* __restrict__ x, i
     s_par[3 * H + c] = beta[c];
   }
   __syncthreads();
+  unsigned long long seed = 0, offset = 0;
+  if (DROP) {
+    seed = (unsigned long long)dr.rng[0];
+    offset = (unsigned long long)dr.rng[1];
+  }
   const int vpr = H >> 2;
   const long long total = N * vpr;
   for (long long id0 = (long long)blockIdx.x * blockDim.x + threadIdx.x; id0 < total;
@@ -209,18 +218,29 @@ __global__ void __launch_bounds__(256) k_bn_apply(const float* __restrict__ x, i
       o.z = fmaf((v[u].z - mu.z) * rs.z, ga.z, be.z);
       o.w = fmaf((v[u].w - mu.w) * rs.w, ga.w, be.w);
       if (relu) o = f4max(o, f4zero());
+      if (DROP) {
+        const uint4 wd = dropout_words(seed, offset, dr.layer, (unsigned long long)id);
+        o.x = wd.x >= dr.t ? o.x * dr.scale : 0.f;
+        o.y = wd.y >= dr.t ? o.y * dr.scale : 0.f;
+        o.z = wd.z >= dr.t ? o.z * dr.scale : 0.f;
+        o.w = wd.w >= dr.t ? o.w * dr.scale : 0.f;
+      }
       st4(y + (size_t)(id / vpr) * ld_y + c, o);
     }
   }
 }
 
-// sums[0:H] += sum_n dz,  sums[H:2H] += sum_n dz*xhat   with dz = dy * (y > 0 if relu)
+// sums[0:H] += sum_n dz,  sums[H:2H] += sum_n dz*xhat   with dz = dy * (y > 0 if relu) * scale.
+// scale = the dropout scale 1/(1-p) of the forward (1 without dropout: then dz is dy bit for bit): y = relu(.) keep scale,
+// so for scale >= 1, y > 0 <=> (kept and relu active) and the saved output is the only mask needed.  SCALED = false: the
+// kernel without the multiply (its register budget, and so its occupancy, is that of the plain kernel).
+template <bool SCALED>
 __global__ void __launch_bounds__(256) k_bn_bwd_reduce(const float* __restrict__ dy, int ld_dy,
                                                         const float* __restrict__ y, int ld_y,
                                                         const float* __restrict__ x, int ld_x,
                                                         const float* __restrict__ mean,
                                                         const float* __restrict__ rstd, long long N, int H, int relu,
-                                                        float* __restrict__ sums) {
+                                                        float scale, float* __restrict__ sums) {
   extern __shared__ float sm[];  // [rl_n][2H]
   const int vpr = H >> 2;
   const int rl_n = blockDim.x / vpr;
@@ -246,6 +266,7 @@ __global__ void __launch_bounds__(256) k_bn_bwd_reduce(const float* __restrict__
         const float4 yy = yy4[u], v = vv[u];
         g.x = yy.x > 0.f ? g.x : 0.f; g.y = yy.y > 0.f ? g.y : 0.f;
         g.z = yy.z > 0.f ? g.z : 0.f; g.w = yy.w > 0.f ? g.w : 0.f;
+        if (SCALED) g = f4scale(scale, g);
         s1 = f4add(s1, g);
         s2.x = fmaf(g.x, (v.x - mu.x) * rs.x, s2.x); s2.y = fmaf(g.y, (v.y - mu.y) * rs.y, s2.y);
         s2.z = fmaf(g.z, (v.z - mu.z) * rs.z, s2.z); s2.w = fmaf(g.w, (v.w - mu.w) * rs.w, s2.w);
@@ -267,7 +288,7 @@ __global__ void k_bn_bwd_apply(const float* __restrict__ dy, int ld_dy, const fl
                                const float* __restrict__ x, int ld_x, const float* __restrict__ mean,
                                const float* __restrict__ rstd, const float* __restrict__ gamma,
                                const float* __restrict__ sums, float* __restrict__ dx, int ld_dx, long long N, int H,
-                               int relu, int training, float* dgamma, float* dbeta) {
+                               int relu, float scale, int training, float* dgamma, float* dbeta) {
   const int vpr = H >> 2;
   long long id = (long long)blockIdx.x * blockDim.x + threadIdx.x;
   if (blockIdx.x == 0)  // parameter grads accumulate (+=) like autograd
@@ -283,6 +304,7 @@ __global__ void k_bn_bwd_apply(const float* __restrict__ dy, int ld_dy, const fl
     float4 yy = ldg4(y + (size_t)n * ld_y + c);
     g.x = yy.x > 0.f ? g.x : 0.f; g.y = yy.y > 0.f ? g.y : 0.f;
     g.z = yy.z > 0.f ? g.z : 0.f; g.w = yy.w > 0.f ? g.w : 0.f;
+    if (scale != 1.f) g = f4scale(scale, g);     // dropout (see k_bn_bwd_reduce)
   }
   const float4 rs = ldg4(rstd + c), ga = ldg4(gamma + c);
   float4 o;
@@ -298,6 +320,17 @@ __global__ void k_bn_bwd_apply(const float* __restrict__ dy, int ld_dy, const fl
     o = make_float4(ga.x * rs.x * g.x, ga.y * rs.y * g.y, ga.z * rs.z * g.z, ga.w * rs.w * g.w);
   }
   st4(dx + (size_t)n * ld_dx + c, o);
+}
+
+// keep[n, c] = 1 iff unit (n, c) of BatchNorm `layer` survives dropout (the mask k_bn_apply<true> applies)
+__global__ void k_dropout_mask(unsigned long long seed, unsigned long long offset, int layer, long long N, int H,
+                               unsigned long long t, uint8_t* __restrict__ keep) {
+  const long long j = (long long)blockIdx.x * blockDim.x + threadIdx.x;
+  if (j >= N * (H >> 2)) return;
+  const uint4 wd = dropout_words(seed, offset, layer, (unsigned long long)j);
+  uchar4 k;
+  k.x = wd.x >= t; k.y = wd.y >= t; k.z = wd.z >= t; k.w = wd.w >= t;
+  reinterpret_cast<uchar4*>(keep)[j] = k;
 }
 
 // ---------------------------------------------------------------- local head + weighted add-pool
@@ -573,20 +606,40 @@ int pert_bn_fwd(const float* x, int ld_x, const float* gamma, const float* beta,
                 int relu, float* mean, float* rstd, float* y, int ld_y, long long N, int H, void* workspace,
                 long long workspace_bytes, void* stream) {
   return pert_bn_fwd_ex(x, ld_x, gamma, beta, running_mean, running_var, num_batches_tracked, eps, momentum, training,
-                        relu, mean, rstd, y, ld_y, N, H, workspace, workspace_bytes, 0, stream);
+                        relu, mean, rstd, y, ld_y, N, H, workspace, workspace_bytes, 0, 0.f, nullptr, 0, stream);
+}
+
+int pert_dropout_mask(long long seed, long long offset, int layer, long long N, int H, float p, uint8_t* keep,
+                      void* stream) {
+  unsigned long long t;
+  float scale;
+  if (!pert_dropout_params(p, &t, &scale)) return PERT_ERR_BADARG;
+  if (N < 0 || H <= 0 || H % 4 || !keep || ((uintptr_t)keep & 3)) return PERT_ERR_BADARG;
+  if (N == 0) return PERT_OK;
+  k_dropout_mask<<<pert_cdiv(N * (H / 4), 256), 256, 0, (cudaStream_t)stream>>>(
+      (unsigned long long)seed, (unsigned long long)offset, layer, N, H, t, keep);
+  PERT_LAUNCH_CHECK();
+  return PERT_OK;
 }
 
 }  // extern "C"
 
 // stats_ready != 0 (training): the fp64 column sums / sums of squares already sit in `workspace` (written by the producer
 // of x, csrc/tconv_tile.cu) -- only the apply pass runs.
+// training with dropout_p > 0: y = relu(bn(x)) * keep / (1 - dropout_p), keep from the device (seed, offset) at
+// rng_state and the BatchNorm index `layer` (see dropout_words); rng_state is only read.  Otherwise dropout is off.
 int pert_bn_fwd_ex(const float* x, int ld_x, const float* gamma, const float* beta, float* running_mean,
                    float* running_var, long long* num_batches_tracked, float eps, float momentum, int training,
                    int relu, float* mean, float* rstd, float* y, int ld_y, long long N, int H, void* workspace,
-                   long long workspace_bytes, int stats_ready, void* stream) {
+                   long long workspace_bytes, int stats_ready, float dropout_p, const long long* rng_state, int layer,
+                   void* stream) {
   if (N < 0 || H <= 0 || H % 4 || H > 1024 || ld_x % 4 || ld_y % 4 || !x || !gamma || !beta || !mean || !rstd || !y)
     return PERT_ERR_BADARG;
   if (!al16(x) || !al16(gamma) || !al16(beta) || !al16(mean) || !al16(rstd) || !al16(y)) return PERT_ERR_BADARG;
+  PertDropout dr{rng_state, 0, 1.f, layer};
+  if (!pert_dropout_params(dropout_p, &dr.t, &dr.scale)) return PERT_ERR_BADARG;
+  const bool drop = training && dropout_p > 0.f;
+  if (drop && !rng_state) return PERT_ERR_BADARG;
   if (N == 0) return PERT_OK;
   cudaStream_t st = (cudaStream_t)stream;
   double* acc = nullptr;
@@ -614,10 +667,16 @@ int pert_bn_fwd_ex(const float* x, int ld_x, const float* gamma, const float* be
   long long total = N * (H / 4);
   long long blocks = pert_cdiv(total, 256 * 4);
   if (blocks > 8LL * PERT_NUM_SMS) blocks = 8LL * PERT_NUM_SMS;
-  k_bn_apply<<<(int)blocks, 256, (size_t)4 * H * sizeof(float), st>>>(x, ld_x, mean, rstd, gamma, beta, y, ld_y, N, H, relu, acc, eps,
-                                                              momentum, training ? running_mean : nullptr,
-                                                              training ? running_var : nullptr,
-                                                              training ? num_batches_tracked : nullptr);
+  const size_t smem = (size_t)4 * H * sizeof(float);
+  float* rm = training ? running_mean : nullptr;
+  float* rv = training ? running_var : nullptr;
+  long long* nbt = training ? num_batches_tracked : nullptr;
+  if (drop)
+    k_bn_apply<true><<<(int)blocks, 256, smem, st>>>(x, ld_x, mean, rstd, gamma, beta, y, ld_y, N, H, relu, acc, eps,
+                                                     momentum, rm, rv, nbt, dr);
+  else
+    k_bn_apply<false><<<(int)blocks, 256, smem, st>>>(x, ld_x, mean, rstd, gamma, beta, y, ld_y, N, H, relu, acc,
+                                                      eps, momentum, rm, rv, nbt, dr);
   PERT_LAUNCH_CHECK();
   return PERT_OK;
 }
@@ -628,8 +687,19 @@ extern "C" {
 int pert_bn_bwd(const float* dy, int ld_dy, const float* y, int ld_y, const float* x, int ld_x, const float* mean,
                 const float* rstd, const float* gamma, int relu, int training, float* dx, int ld_dx, float* dgamma,
                 float* dbeta, float* sums, long long N, int H, void* stream) {
+  return pert_bn_bwd_ex(dy, ld_dy, y, ld_y, x, ld_x, mean, rstd, gamma, relu, training, 1.f, dx, ld_dx, dgamma, dbeta,
+                        sums, N, H, stream);
+}
+
+}  // extern "C"
+
+// dropout_scale: 1/(1-p) of a training forward that applied dropout to y (relu only), else 1.
+int pert_bn_bwd_ex(const float* dy, int ld_dy, const float* y, int ld_y, const float* x, int ld_x, const float* mean,
+                   const float* rstd, const float* gamma, int relu, int training, float dropout_scale, float* dx,
+                   int ld_dx, float* dgamma, float* dbeta, float* sums, long long N, int H, void* stream) {
   if (N < 0 || H <= 0 || H % 4 || H > 1024 || !dy || !x || !mean || !rstd || !gamma || !dx || !sums)
     return PERT_ERR_BADARG;
+  if (dropout_scale != 1.f && !(relu && dropout_scale >= 0.f)) return PERT_ERR_BADARG;
   if (relu && !y) return PERT_ERR_BADARG;
   if (ld_dy % 4 || ld_x % 4 || ld_dx % 4 || (relu && ld_y % 4)) return PERT_ERR_BADARG;
   if (!al16(dy) || !al16(y) || !al16(x) || !al16(mean) || !al16(rstd) || !al16(gamma) || !al16(dx) || !al16(sums))
@@ -644,14 +714,20 @@ int pert_bn_bwd(const float* dy, int ld_dy, const float* y, int ld_y, const floa
   int rl_n = threads / vpr;
   size_t smem = (size_t)rl_n * 2 * H * sizeof(float);
   if (smem > 48 * 1024) return PERT_ERR_UNSUPPORTED;
-  k_bn_bwd_reduce<<<pert_cdiv(N, BN_BWD_ROWS), threads, smem, st>>>(dy, ld_dy, y, ld_y, x, ld_x, mean, rstd, N, H, relu,
-                                                              sums);
+  if (dropout_scale != 1.f)
+    k_bn_bwd_reduce<true><<<pert_cdiv(N, BN_BWD_ROWS), threads, smem, st>>>(dy, ld_dy, y, ld_y, x, ld_x, mean, rstd, N,
+                                                                           H, relu, dropout_scale, sums);
+  else
+    k_bn_bwd_reduce<false><<<pert_cdiv(N, BN_BWD_ROWS), threads, smem, st>>>(dy, ld_dy, y, ld_y, x, ld_x, mean, rstd,
+                                                                            N, H, relu, 1.f, sums);
   long long total = N * vpr;
   k_bn_bwd_apply<<<pert_cdiv(total, 256), 256, 0, st>>>(dy, ld_dy, y, ld_y, x, ld_x, mean, rstd, gamma, sums, dx,
-                                                       ld_dx, N, H, relu, training, dgamma, dbeta);
+                                                       ld_dx, N, H, relu, dropout_scale, training, dgamma, dbeta);
   PERT_LAUNCH_CHECK();
   return PERT_OK;
 }
+
+extern "C" {
 
 // local[n] = <x_n, w_local> + b_local (optional);  pool[batch[n]] += x_n * probs[n] / pnn[n]  (pool zeroed here)
 int pert_pool_fwd(const float* x, int ld, const float* probs, const float* pnn, const int64_t* batch,

@@ -40,7 +40,7 @@ class PertProbe(C.Structure):
     """Measurement probe (include/pertgnn.h): two CUDA events recorded around one kernel family of one layer."""
     _fields_ = [("kernel", C.c_int32), ("layer", C.c_int32), ("ev_start", C.c_void_p), ("ev_stop", C.c_void_p)]
 
-    KERNELS = {"tconv_fwd": 1, "tconv_bwd": 2, "gemm_fwd": 3, "gemm_wgrad": 4, "gemm_dgrad": 5}
+    KERNELS = {"tconv_fwd": 1, "tconv_bwd": 2, "gemm_fwd": 3, "gemm_wgrad": 4, "gemm_dgrad": 5, "bn_apply": 6}
     _rt = None
 
     @classmethod
@@ -141,6 +141,11 @@ class Engine:
         self.ws_key = (0, 0, 0)
         self.ws_generation = 0
         self._saved = None
+        # dropout generator state (seed, offset), read by the BatchNorm kernels; every training forward with p > 0 adds 1
+        # to the offset on the device (so a replayed CUDA graph draws fresh masks).  The seed is drawn from torch's
+        # default generator at the first forward that needs it: a model without dropout never consumes random numbers.
+        self.rng = torch.zeros(2, device=dev, dtype=torch.int64)
+        self._rng_seeded = False
 
     # ------------------------------------------------------------------------------------------
     @property
@@ -164,10 +169,38 @@ class Engine:
             self.ws_generation += 1
         return self.ws
 
+    def seed_dropout(self, seed, offset=0):
+        """Sets the dropout generator state: the masks of a forward are a function of (seed, offset, layer) only."""
+        seed = int(seed) & 0xFFFFFFFFFFFFFFFF
+        if seed >= 1 << 63:
+            seed -= 1 << 64                                  # the same 64 bits as an int64
+        with torch.cuda.device(self.device):
+            self.rng.copy_(torch.tensor([seed, int(offset)], dtype=torch.int64))
+        self._rng_seeded = True
+
+    @_lib.on_device_of
+    def dropout_masks(self):
+        """{'bn{i}': [N,H] bool}: the dropout keep masks of the LAST forward (all True when it applied no dropout), from
+        pert_dropout_mask with the offset that forward used (read back from the device state).  Test aid, like
+        ``active_relus``."""
+        x, cat_X, entry_id, probs, pnn, batch, index, training, N, E, B, p = self._saved
+        H = self.desc.H
+        if not (training and p > 0):
+            return {f"bn{l}": torch.ones(N, H, dtype=torch.bool, device=self.device) for l in range(self.n_convs - 1)}
+        seed, offset = self.rng.tolist()
+        out = {}
+        for l in range(self.n_convs - 1):
+            keep = torch.empty(N, H, dtype=torch.uint8, device=self.device)
+            _lib.check(self.lib.pert_dropout_mask(seed, offset - 1, l, N, H, p, _lib.ptr(keep), _lib.stream()),
+                       "pert_dropout_mask")
+            out[f"bn{l}"] = keep.bool()
+        return out
+
     def active_relus(self):
         """{'bn{i}': [N,H] bool, 'head': [B,H] bool}: which ReLUs were active in the LAST forward (read from the saved
-        activations in the workspace).  Test aid: lets a reference be differentiated on the same linear piece."""
-        x, cat_X, entry_id, probs, pnn, batch, index, training, N, E, B = self._saved
+        activations in the workspace; with dropout, a dropped unit reads as inactive).  Test aid: lets a reference be
+        differentiated on the same linear piece."""
+        x, cat_X, entry_id, probs, pnn, batch, index, training, N, E, B, p = self._saved
         H = self.desc.H
         out = {}
         for l in range(1, self.n_convs):
@@ -191,7 +224,7 @@ class Engine:
     def launches_forward(self):
         """Kernels pert_model_forward launches (memsets not counted): pack, edge tables (6 layers per launch),
         embeddings + copy, per conv GEMM + attention (whose epilogue also produces the BatchNorm statistics), per
-        BatchNorm one apply kernel, pool, head."""
+        BatchNorm one apply kernel (dropout included), pool, head (which also advances the dropout offset)."""
         L = self.n_convs
         return self._pack_launches() + (L + 5) // 6 + self.desc.n_cat + 1 + 2 * L + (L - 1) + 1 + 1
 
@@ -204,8 +237,13 @@ class Engine:
     @_lib.on_device_of
     def forward(self, x, cat_X, entry_id, probs, pnn, batch, index: GraphIndex, training, probe=None,
                 index_ready=None):
-        """-> (global_pred [B,1], local_pred [N,1]); keeps what backward needs in the workspace."""
+        """-> (global_pred [B,1], local_pred [N,1]); keeps what backward needs in the workspace.  Training with
+        ``model.dropout > 0`` applies dropout after every BatchNorm+ReLU (masks from ``self.rng``)."""
         N, E, B = x.size(0), index.E, entry_id.numel()
+        p_drop = float(self.model.dropout)
+        drop = bool(training) and p_drop > 0
+        if drop and not self._rng_seeded:
+            self.seed_dropout(int(torch.empty((), dtype=torch.int64).random_()))
         ws = self._workspace(N, E, B)
         dev = x.device
         x = x.contiguous().float()
@@ -220,18 +258,19 @@ class Engine:
         rc = self.lib.pert_model_forward(
             C.byref(self.desc), p(self.fp.flat), p(self.bn_running), p(self.bn_nbt), p(x), p(cat_X), p(entry_id),
             p(probs), p(pnn), p(batch), N, E, B, p(index.rowptr), p(index.csr_src), p(index.csr_if), p(index.csr_rpc),
-            p(ws), ws.numel() * 4, int(training), p(gpred), p(lpred), p(index.status),
+            p(ws), ws.numel() * 4, int(training), p_drop, p(self.rng) if drop else None, p(gpred), p(lpred),
+            p(index.status),
             C.byref(probe) if probe is not None else None,
             C.c_void_p(index_ready.cuda_event) if index_ready is not None else None, _lib.stream())
         _lib.check(rc, "pert_model_forward")
         ops.LAUNCHES["n"] += self.launches_forward()
-        self._saved = (x, cat_X, entry_id, probs, pnn, batch, index, bool(training), N, E, B)
+        self._saved = (x, cat_X, entry_id, probs, pnn, batch, index, bool(training), N, E, B, p_drop)
         return gpred, lpred
 
     @_lib.on_device_of
     def backward(self, d_global, d_local=None, grads=None, probe=None):
         """Accumulates (+=) parameter gradients into ``grads`` (default: the flat gradient buffer)."""
-        x, cat_X, entry_id, probs, pnn, batch, index, training, N, E, B = self._saved
+        x, cat_X, entry_id, probs, pnn, batch, index, training, N, E, B, p_drop = self._saved
         grads = self.fp.grad if grads is None else grads
         d_global = d_global.reshape(-1).contiguous().float()
         if d_local is not None:
@@ -241,7 +280,7 @@ class Engine:
         rc = self.lib.pert_model_backward(
             C.byref(self.desc), p(self.fp.flat), p(grads), p(cat_X), p(entry_id), p(probs), p(pnn), p(batch), N, E, B,
             p(index.rowptr), p(index.csr_src), p(index.csr_if), p(index.csr_rpc), p(index.colptr), p(index.csc_pos),
-            p(index.csc_dst), p(ws), ws.numel() * 4, int(training), p(d_global), p(d_local),
+            p(index.csc_dst), p(ws), ws.numel() * 4, int(training), p_drop, p(d_global), p(d_local),
             C.byref(probe) if probe is not None else None, _lib.stream())
         _lib.check(rc, "pert_model_backward")
         ops.LAUNCHES["n"] += self.launches_backward()

@@ -40,7 +40,8 @@ class SAGEDeterministic(torch.nn.Module):
         self.rpctype_embeds = torch.nn.Embedding(rpctype_id_max + 1, H)
         self.edge_linear = Linear(-1, 2 * H)   # lazy + unused in the reference forward (model.py:68): bias only
         # True: whole forward/backward issued by the C++ step engine (csrc/engine.cu); False: one autograd
-        # Function per operator (ops.py).  Same kernels, same results; the engine removes the interpreter gaps.
+        # Function per operator (ops.py).  Same kernels, same results; the engine removes the interpreter gaps.  (Dropout:
+        # the engine draws its own counter-based masks, the operator path calls F.dropout -- same distribution.)
         self.use_engine = True
         self._engine = None
         # test hook (operator path only): dict that receives the post-ReLU activations ('bn{i}', 'head'), so that a reference
@@ -82,7 +83,8 @@ class SAGEDeterministic(torch.nn.Module):
             index = cached_index(edge_index, N, edge_attr, self.interface_embeds.num_embeddings,
                                  self.rpctype_embeds.num_embeddings)
         index.num_graphs = entry_id.numel()
-        if self.use_engine and (self.dropout == 0 or not self.training):
+        if self.use_engine:
+            # training dropout (model.py:103) runs inside the engine's BatchNorm kernels (Engine.forward)
             from .engine import engine_forward
 
             return engine_forward(self.engine(), x, cat_X, entry_id, pattern_probs, pattern_num_nodes, batch, index,

@@ -378,7 +378,8 @@ class GraphedTrainStep:
         return loss
 
     def __call__(self, data):
-        key = self._key(data)
+        # the dropout threshold and scale are by-value kernel arguments: frozen in a captured graph
+        key = self._key(data) + (float(self.model.dropout),)
         ent = self._seen.get(key, "unseen")
         if isinstance(ent, dict):
             pass
