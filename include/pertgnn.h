@@ -48,7 +48,8 @@ extern "C" {
 /* ABI version (major*1000 + minor).  2000: pert_tconv_bwd takes rpc_ws; node_depth / eval-metric entry points.
  * 2001: pert_pert_graph_count / pert_pert_graph_build.  2002: pert_allreduce_adam timing[5], reduce-scatter form.
  * 2003: pert_span_graph_count / pert_span_graph_build.  2004: training-mode dropout in the step engine
- * (pert_model_forward gains dropout_p + rng_state, pert_model_backward gains dropout_p), pert_dropout_mask. */
+ * (pert_model_forward gains dropout_p + rng_state, pert_model_backward gains dropout_p), pert_dropout_mask.
+ * 2005: pert_catalogue_* (trace catalogue). */
 int pert_version(void);
 
 /* ---- index construction (integer, bit-exact) ---------------------------------------------------
@@ -379,6 +380,54 @@ int pert_span_graph_build(const int64_t* row_ptr, long long T, long long R, cons
                           const int64_t* interface, const int64_t* rpctype, const int64_t* root_ms,
                           const int64_t* node_ptr, int max_rows, int global_ids, int64_t* ms_id, int64_t* edge_index,
                           int64_t* edge_attr, int64_t* root_nid, int* status, void* stream);
+
+/* ---- trace catalogue (csrc/catalogue.cu; Python: pert_gnn_kdd23_b200/catalogue.py) -------------------------------
+ * Replaces the integer-coded part of preprocess.py:main() (:269-375): the per-trace pattern strings and their
+ * factorize (:280-293), tr2ts_map (:39), tr2delay (:290-292), the per-entry Python loop (:295-367) and the
+ * normalisation (:371-375).  All arrays int64 unless stated.  Traces are numbered by ascending traceid; `perm[R]` is
+ * the row order grouped by traceid (stable, file order inside a trace), row_ptr[T+1] its trace offsets.
+ *
+ * run_flags: flag[i] = (i == 0 || key[i] != key[i-1]); mark[i] = flag[i] ? i : 0 (mark may be NULL). */
+int pert_catalogue_run_flags(const int64_t* key, long long n, int64_t* flag, int64_t* mark, void* stream);
+/* Per trace (one warp each, no row limit): nrows, hash = order-sensitive 64-bit hash of the (um, dm, interface) row
+ * sequence (:280-289) & hash_mask, y = max |rt| (:290-292), ts_bucket = floor(min timestamp / 30000) * 30000 (:39),
+ * trace_entry = entryid of the first row; PERT_ERR_RANGE in status if the trace's rows carry different entryids. */
+int pert_catalogue_summary(const int64_t* perm, const int64_t* row_ptr, long long T, const int64_t* um,
+                           const int64_t* dm, const int64_t* interface, const int64_t* rt, const int64_t* timestamp,
+                           const int64_t* entryid, unsigned long long seed, unsigned long long hash_mask,
+                           int64_t* nrows, int64_t* hash, int64_t* y, int64_t* ts_bucket, int64_t* trace_entry,
+                           int* status, void* stream);
+/* Exact check of a grouping by key (:293 factorize compares the strings): order[T] = traces sorted by (key, trace),
+ * head[i] = sorted position of the first member of i's run.  mismatch[order[i]] = 1 iff that trace's sequence differs
+ * from its head's; n_mismatch (device uint64, zeroed by the call) counts them. */
+int pert_catalogue_verify(const int64_t* order, const int64_t* head, long long T, const int64_t* perm,
+                          const int64_t* row_ptr, const int64_t* um, const int64_t* dm, const int64_t* interface,
+                          int32_t* mismatch, unsigned long long* n_mismatch, void* stream);
+/* For every trace with mismatch[t]: key[t] = mix(key[t], sequence hash with `seed` & hash_mask). */
+int pert_catalogue_rekey(const int64_t* perm, const int64_t* row_ptr, long long T, const int64_t* um,
+                         const int64_t* dm, const int64_t* interface, const int32_t* mismatch, unsigned long long seed,
+                         unsigned long long hash_mask, int64_t* key, void* stream);
+/* canon[order[i]] = order[head[i]] (first trace of the pattern), first[t] = (canon[t] == t). */
+int pert_catalogue_canon(const int64_t* order, const int64_t* head, long long T, int64_t* canon, int64_t* first,
+                         void* stream);
+/* rid[t] = first_incl[canon[t]] - 1 (first_incl = inclusive scan of `first`): runtime ids in factorize order (:293). */
+int pert_catalogue_runtime_ids(const int64_t* canon, const int64_t* first_incl, long long T, int64_t* rid,
+                               void* stream);
+/* eorder[T] = traces in (entry, traceid) order (the order of :295-299), eidx[j] = rank of the entry of eorder[j].
+ * Per pattern (P of them): rep_epos = smallest j showing it (its representative, :317-318), occurrences (:342);
+ * pair_key[j] = eidx[j] * P + rid[eorder[j]]. */
+int pert_catalogue_patterns(const int64_t* eorder, const int64_t* eidx, long long T, const int64_t* rid, long long P,
+                            int64_t* rep_epos, int64_t* occurrences, int64_t* pair_key, void* stream);
+/* (entry, pattern) pairs (:310-316): pstart[NP] = run starts of the stably sorted pair_key, pidx[T] its sort indices.
+ * Per pair: count, first = entry-order position of its first trace, pair_entry (entry rank), pair_rid. */
+int pert_catalogue_pairs(const int64_t* pstart, long long NP, long long T, const int64_t* pidx, const int64_t* eorder,
+                         const int64_t* rid, const int64_t* eidx, int64_t* count, int64_t* first, int64_t* pair_entry,
+                         int64_t* pair_rid, void* stream);
+/* Pairs sorted by `first` (entry-major, then first appearance): prob (double) = count / traces of the entry
+ * (:371-375, bit-identical to Python's int / int), ent_ptr[E+1] = the entry CSR over the pairs; ent_start[E] = first
+ * entry-order position of every entry. */
+int pert_catalogue_probs(const int64_t* pair_entry, const int64_t* count, long long NP, const int64_t* ent_start,
+                         long long E, long long T, double* prob, int64_t* ent_ptr, void* stream);
 
 #ifdef __cplusplus
 }

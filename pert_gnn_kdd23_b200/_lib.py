@@ -14,7 +14,7 @@ import torch
 _HERE = os.path.dirname(os.path.abspath(__file__))
 LIB_PATH = os.path.join(_HERE, "libpertgnn.so")
 
-P, I, LL, F = C.c_void_p, C.c_int, C.c_longlong, C.c_float
+P, I, LL, F, ULL = C.c_void_p, C.c_int, C.c_longlong, C.c_float, C.c_ulonglong
 
 # name -> (restype, argtypes); must mirror include/pertgnn.h
 SIGNATURES = {
@@ -68,6 +68,16 @@ SIGNATURES = {
                                P]),
     "pert_model_backward": (I, [P, P, P, P, P, P, P, P, LL, LL, LL, P, P, P, P, P, P, P, P, LL, I, F, P, P, P, P]),
     "pert_dropout_mask": (I, [LL, LL, I, LL, I, F, P, P]),
+    # trace catalogue (catalogue.py)
+    "pert_catalogue_run_flags": (I, [P, LL, P, P, P]),
+    "pert_catalogue_summary": (I, [P, P, LL, P, P, P, P, P, P, ULL, ULL, P, P, P, P, P, P, P]),
+    "pert_catalogue_verify": (I, [P, P, LL, P, P, P, P, P, P, P, P]),
+    "pert_catalogue_rekey": (I, [P, P, LL, P, P, P, P, ULL, ULL, P, P]),
+    "pert_catalogue_canon": (I, [P, P, LL, P, P, P]),
+    "pert_catalogue_runtime_ids": (I, [P, P, LL, P, P]),
+    "pert_catalogue_patterns": (I, [P, P, LL, P, LL, P, P, P, P]),
+    "pert_catalogue_pairs": (I, [P, LL, LL, P, P, P, P, P, P, P, P, P]),
+    "pert_catalogue_probs": (I, [P, P, LL, P, LL, LL, P, P, P]),
 }
 
 _lib = None

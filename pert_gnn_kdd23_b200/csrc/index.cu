@@ -339,7 +339,7 @@ __global__ void k_graph_ptr_count(const int64_t* __restrict__ batch, int N, int 
 
 extern "C" {
 
-int pert_version(void) { return 2004; }
+int pert_version(void) { return 2005; }
 
 long long pert_index_workspace_bytes(long long N, long long E) {
   if (N < 0 || E < 0) return PERT_ERR_BADARG;

@@ -60,6 +60,21 @@ class _BulkPatterns:
         self.ms_id, self.node_depth, self.edge_index, self.edge_attr = ms_id, node_depth, edge_index, edge_attr
 
 
+class _EntryCSR:
+    """entry2runtimes as arrays over entry ids 0..n_ent-1 (PatternStore.from_catalogue): ent_ptr [n_ent+1], ent_pat
+    (pattern index), ent_prob (float64)."""
+
+    def __init__(self, ent_ptr, ent_pat, ent_prob):
+        self.ent_ptr, self.ent_pat, self.ent_prob = ent_ptr, ent_pat, ent_prob
+
+
+class _TraceArrays:
+    """tr2data as arrays in its dict order (PatternStore.from_catalogue): keys, entry, ts, y."""
+
+    def __init__(self, keys, entry, ts, y):
+        self.keys, self.entry, self.ts, self.y = keys, entry, ts, y
+
+
 class PatternStore:
     """Patterns, entries, resource table and traces on one CUDA device."""
 
@@ -112,17 +127,25 @@ class PatternStore:
         pat_nodes = np.diff(nptr)
         pat_edges = np.diff(eptr)
         # ---- entries, in the dict order of entry2runtimes[entry] (get_all_runtimes_id_probs, pert_gnn.py:70-74)
-        n_ent = max(entry2runtimes.keys()) + 1
-        ent_ptr, ent_pat, ent_prob = [0], [], []
-        ent_nodes, ent_edges = np.zeros(n_ent, dtype=np.int32), np.zeros(n_ent, dtype=np.int32)
-        for e in range(n_ent):
-            for rt, pr in entry2runtimes.get(e, {}).items():
-                k = rt_index[rt]
-                ent_pat.append(k)
-                ent_prob.append(pr)
-                ent_nodes[e] += pat_nodes[k]
-                ent_edges[e] += pat_edges[k]
-            ent_ptr.append(len(ent_pat))
+        if isinstance(entry2runtimes, _EntryCSR):
+            ec = entry2runtimes
+            n_ent = len(ec.ent_ptr) - 1
+            ent_ptr, ent_pat, ent_prob = ec.ent_ptr, ec.ent_pat, ec.ent_prob
+            pe = np.repeat(np.arange(n_ent), np.diff(ent_ptr))
+            ent_nodes = np.bincount(pe, weights=pat_nodes[ent_pat], minlength=n_ent).astype(np.int32)
+            ent_edges = np.bincount(pe, weights=pat_edges[ent_pat], minlength=n_ent).astype(np.int32)
+        else:
+            n_ent = max(entry2runtimes.keys()) + 1
+            ent_ptr, ent_pat, ent_prob = [0], [], []
+            ent_nodes, ent_edges = np.zeros(n_ent, dtype=np.int32), np.zeros(n_ent, dtype=np.int32)
+            for e in range(n_ent):
+                for rt, pr in entry2runtimes.get(e, {}).items():
+                    k = rt_index[rt]
+                    ent_pat.append(k)
+                    ent_prob.append(pr)
+                    ent_nodes[e] += pat_nodes[k]
+                    ent_edges[e] += pat_edges[k]
+                ent_ptr.append(len(ent_pat))
         res_ms = np.array([m for _, m in resource_index], dtype=np.int64)
         res_ts = np.array([t for t, _ in resource_index], dtype=np.int64)
         self.n_ms = int(n_ms if n_ms is not None else max(int(all_ms.max(initial=0)), int(res_ms.max(initial=0))) + 1)
@@ -131,10 +154,14 @@ class PatternStore:
         has = np.zeros(self.n_ms, dtype=np.uint8)
         has[res_ms] = 1                                          # ms_with_resources (pert_gnn.py:138)
         # ---- traces, in the dict order of tr2data (get_data_list, pert_gnn.py:176-188)
-        self.trace_keys = list(tr2data.keys())
-        t_ent = np.array([int(tr2data[k]["entry_id"]) for k in self.trace_keys], dtype=np.int32)
-        t_ts = np.array([int(tr2data[k]["timestamp"]) for k in self.trace_keys], dtype=np.int64)
-        t_y = np.array([int(tr2data[k]["y"]) for k in self.trace_keys], dtype=np.int64)
+        if isinstance(tr2data, _TraceArrays):
+            self.trace_keys = tr2data.keys
+            t_ent, t_ts, t_y = tr2data.entry.astype(np.int32), tr2data.ts, tr2data.y
+        else:
+            self.trace_keys = list(tr2data.keys())
+            t_ent = np.array([int(tr2data[k]["entry_id"]) for k in self.trace_keys], dtype=np.int32)
+            t_ts = np.array([int(tr2data[k]["timestamp"]) for k in self.trace_keys], dtype=np.int64)
+            t_y = np.array([int(tr2data[k]["y"]) for k in self.trace_keys], dtype=np.int64)
         # host copies used to size the outputs without a device sync
         self._h_ent_nodes, self._h_ent_edges = ent_nodes.astype(np.int64), ent_edges.astype(np.int64)
         self._h_ent_pats = np.diff(np.array(ent_ptr)).astype(np.int64)
@@ -179,6 +206,28 @@ class PatternStore:
                            graphs.edge_index.cpu().numpy(), graphs.edge_attr.cpu().numpy())
         assert len(bp.rt_ids) == len(bp.node_ptr) - 1
         return cls(bp, entry2runtimes, resource_index, resource_values, tr2data, dev, n_ms=n_ms)
+
+    @classmethod
+    def from_catalogue(cls, cat, graphs, resource_index, resource_values, device=None, n_ms=None):
+        """Store of a ``catalogue.Catalogue`` (``graphs``: ``cat.graphs(kind)``) without per-trace or per-entry Python
+        dicts: the same device arrays as ``PatternStore(*cat.to_reference(kind), resource_index, resource_values,
+        ...)`` (traces in tr2data order, patterns in runtime2graph order, entries by id)."""
+        h = {k: getattr(cat, k).cpu().numpy() for k in ("traceid", "entry", "timestamp", "y", "pat_runtime_id",
+                                                         "entries", "ent_ptr", "ent_runtime_id", "ent_prob")}
+        pos = np.empty(len(h["pat_runtime_id"]), dtype=np.int64)
+        pos[h["pat_runtime_id"]] = np.arange(len(pos))                 # runtime id -> pattern index
+        n_ent = int(h["entries"].max()) + 1
+        counts = np.zeros(n_ent, dtype=np.int64)
+        counts[h["entries"]] = np.diff(h["ent_ptr"])
+        ent_ptr = np.concatenate([[0], np.cumsum(counts)]).astype(np.int64)
+        entries = _EntryCSR(ent_ptr, pos[h["ent_runtime_id"]], h["ent_prob"])
+        traces = _TraceArrays(h["traceid"].tolist(), h["entry"], h["timestamp"], h["y"])
+        dev = torch.device(device) if device is not None else cat.device
+        bp = _BulkPatterns(h["pat_runtime_id"].tolist(), np.asarray(graphs.node_ptr), np.asarray(graphs.edge_ptr),
+                           graphs.ms_id.cpu().numpy().reshape(-1), graphs.node_depth.cpu().numpy().reshape(-1),
+                           graphs.edge_index.cpu().numpy(), graphs.edge_attr.cpu().numpy())
+        assert len(bp.rt_ids) == len(bp.node_ptr) - 1
+        return cls(bp, entries, resource_index, resource_values, traces, dev, n_ms=n_ms)
 
     @classmethod
     def from_artifacts(cls, art, device):

@@ -325,3 +325,69 @@ def make_pert_artifacts(seed=3, n_patterns=256, n_entries=64, n_traces=4096, cal
     info = {"patterns": len(pg), "span_rows": int(sum(len(t["um"]) for t in tables)), "nodes": int(pg.node_ptr[-1]),
             "edges": int(pg.edge_ptr[-1]), "build_s": secs}
     return art, info
+
+
+RESOURCE_COLUMNS = tuple(f"instance_{k}_usage_{s}" for k in ("cpu", "memory") for s in ("max", "min", "mean", "median"))
+
+
+def make_processed_tables(seed=5, n_traces=300, n_patterns=24, n_entries=8, n_ms=30, rows=(1, 12), n_if=16, n_rpc=4,
+                          traceid_base=0):
+    """Seeded span table in the ``processed/processed_df.csv`` schema (what preprocess.py:main() reads; int64 columns
+    traceid, timestamp, rpcid, um, dm, interface, rpctype, rt, entryid) + the matching ``processed_resource_df.csv``
+    (timestamp, msname, 8 statistics) with a row for every (30 s bucket of a trace, microservice), as main() needs.
+    -> (table: dict of int64 arrays in file order, resource: dict of arrays).
+
+    Patterns are (um, dm, interface) sequences; the traces of one pattern differ in rpctype, rpcid, timestamps and rt.
+    Row 0 of every pattern is the root call (the largest |rt| at the smallest timestamp; its um occurs nowhere else).
+    The table has self loops and repeated rpcids, one pattern under two entries, single-row traces, traces starting
+    next to a 30 s bucket boundary, non-dense traceids (+ ``traceid_base``) and entry ids with gaps; rows are sorted by
+    timestamp (as get_df leaves them), so traces interleave."""
+    rng = np.random.default_rng(seed)
+    pats = []
+    for p in range(n_patterns):
+        L = 1 if p % 7 == 3 else int(rng.integers(rows[0], rows[1] + 1))
+        root, first = 0, int(rng.integers(1, n_ms))
+        seq = [(root, first, int(rng.integers(0, n_if)))]
+        called = [first]
+        for _ in range(L - 1):
+            um = called[int(rng.integers(0, len(called)))]
+            dm = um if rng.random() < 0.08 else int(rng.integers(1, n_ms))            # self loops
+            seq.append((um, dm, int(rng.integers(0, n_if))))
+            called.append(dm)
+        pats.append(np.array(seq, dtype=np.int64))
+    entry_ids = np.sort(rng.choice(np.arange(2, 40), size=n_entries, replace=False)) * 3     # ids with gaps
+    ent_pats = [list(rng.choice(n_patterns, size=int(rng.integers(2, 6)), replace=False)) for _ in range(n_entries)]
+    ent_pats[1].append(int(ent_pats[0][0]))                                         # one pattern under two entries
+    traceids = rng.choice(np.arange(10, 50 * n_traces), size=n_traces, replace=False).astype(np.int64) + traceid_base
+    cols = {k: [] for k in ("traceid", "timestamp", "rpcid", "um", "dm", "interface", "rpctype", "rt", "entryid")}
+    for i, tid in enumerate(traceids):
+        e = int(rng.integers(0, n_entries))
+        seq = pats[int(ent_pats[e][int(rng.integers(0, len(ent_pats[e])))])]
+        n = len(seq)
+        bucket = 30000 * int(rng.integers(1, 6))
+        t0 = bucket + int(rng.choice([-2, -1, 0, 1, 5000, 20000])) if i % 5 == 0 else bucket + int(rng.integers(0, 29000))
+        ts = t0 + np.concatenate([[0], np.sort(rng.integers(0, 900, size=n - 1))]).astype(np.int64)
+        rt = rng.integers(1, 400, size=n) * np.where(rng.random(n) < 0.5, -1, 1)
+        rt[0] = 1000 + int(rng.integers(0, 500))                                    # root: the largest |rt|
+        rpcid = rng.permutation(n).astype(np.int64) + int(rng.integers(0, 1000))
+        if n > 3 and rng.random() < 0.5:
+            rpcid[int(rng.integers(2, n))] = rpcid[1]                                # repeated rpcid
+        cols["traceid"].append(np.full(n, tid))
+        cols["timestamp"].append(ts)
+        cols["rpcid"].append(rpcid)
+        cols["um"].append(seq[:, 0])
+        cols["dm"].append(seq[:, 1])
+        cols["interface"].append(seq[:, 2])
+        cols["rpctype"].append(rng.integers(0, n_rpc, size=n))
+        cols["rt"].append(rt)
+        cols["entryid"].append(np.full(n, entry_ids[e]))
+    table = {k: np.concatenate(v).astype(np.int64) for k, v in cols.items()}
+    order = np.argsort(table["timestamp"], kind="stable")                           # get_df sorts by timestamp
+    table = {k: v[order] for k, v in table.items()}
+    buckets = np.unique(table["timestamp"] // 30000 * 30000)
+    res_ts, res_ms = np.repeat(buckets, n_ms), np.tile(np.arange(n_ms, dtype=np.int64), len(buckets))
+    resource = {"timestamp": res_ts, "msname": res_ms}
+    vals = rng.random((len(res_ts), len(RESOURCE_COLUMNS)))
+    for j, c in enumerate(RESOURCE_COLUMNS):
+        resource[c] = vals[:, j]
+    return table, resource
